@@ -2,6 +2,7 @@
 """bench.py — CenterPoint frames/s on B200 (driver contract, see the task's Measurement rules).
 
   python bench.py [--gpus N] [--steps K] [--warmup W]            this repo's CUDA path
+                 [--dump-outputs DIR]                            + what the last timed step computed, as DIR/*.npy
   python bench.py --impl reference [--steps K] [--warmup W]      the reference's CPU arm on the host cores
 
 A step = one synthetic nuScenes-shaped frame (300k x 5 points, 1440 x 1440 x 40 grid, max 160000 voxels) through the
@@ -286,9 +287,9 @@ def dense_flops(net, H, W):
     return total
 
 
-def measure(sweep, dev_frames, host_frames, args, world, dist, sample_clocks, local):
+def measure(sweep, dev_frames, host_frames, args, world, dist, sample_clocks, local, keep_outputs=False):
     """Device-timed resident-input rate, e2e (pipelined and one-frame-at-a-time) for one sweep engine (len(sweep) frames in
-    flight, CenterPointSweep).  Returns a dict."""
+    flight, CenterPointSweep).  Returns a dict; keep_outputs adds "outputs", the results of the last timed step."""
     import torch
     pipe = sweep.lanes[0]
     st = pipe.stream
@@ -324,6 +325,7 @@ def measure(sweep, dev_frames, host_frames, args, world, dist, sample_clocks, lo
     barrier()
     wall = time.perf_counter() - t0
     dev_ms = s.elapsed_time(e)
+    outputs = last_step_outputs(sweep.lanes[(args.steps - 1) % len(sweep)]) if keep_outputs else None
     # ---- e2e through the public API (host in, host out), same K
     sweep.prepare_sweep()
     for i in range(3):
@@ -350,7 +352,18 @@ def measure(sweep, dev_frames, host_frames, args, world, dist, sample_clocks, lo
     dev_ms, e2e_ms, wall_ms, sync_ms = [float(x) for x in tt.cpu()]
     total = args.steps * world
     return {"value": total / (dev_ms * 1e-3), "ms_per_step": dev_ms / args.steps, "e2e_value": total / (e2e_ms * 1e-3),
-            "e2e_sync_value": total / (sync_ms * 1e-3), "wall_ms_per_step": wall_ms / args.steps, "clocks": clocks}
+            "e2e_sync_value": total / (sync_ms * 1e-3), "wall_ms_per_step": wall_ms / args.steps, "clocks": clocks,
+            "outputs": outputs}
+
+
+def last_step_outputs(lane):
+    """What CenterPointHotPath.infer hands its caller for the frame `lane` computed last (boxes [K, 9], scores [K],
+    labels [K]) plus the per-task box counts, as float32 / float64 numpy arrays (labels and counts are small integers)."""
+    o = {k: lane.out[k].cpu() for k in ("boxes", "scores", "labels", "counts", "status")}
+    lane.check_status(o["status"])
+    k = int(o["counts"][-1])
+    return {"boxes": o["boxes"][:k].numpy().astype(np.float32), "scores": o["scores"][:k].numpy().astype(np.float32),
+            "labels": o["labels"][:k].numpy().astype(np.float64), "counts": o["counts"].numpy().astype(np.float64)}
 
 
 def reference_gpu_race(dev, stream):
@@ -433,6 +446,8 @@ def main():
     ap.add_argument("--no-head", action="store_true", help="skip the dense RPN / neck / CenterHead (round-1 workload)")
     ap.add_argument("--no-second-geometry", action="store_true")
     ap.add_argument("--in-flight", type=int, default=4, help="frames computing concurrently per GPU (CenterPointSweep lanes)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed (boxes, scores, labels, "
+                    "per-task counts of rank 0) to DIR/<name>.npy; the inputs depend only on the arguments")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
@@ -481,7 +496,11 @@ def main():
         p.capture()
     graph_nodes = pipe.graph_nodes["kernel"] if (rank == 0 and pipe.graph_nodes) else None
     st = pipe.stream
-    m = measure(sweep, dev_frames, host_frames, args, world, dist, True, local)
+    m = measure(sweep, dev_frames, host_frames, args, world, dist, True, local, keep_outputs=bool(args.dump_outputs))
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in m["outputs"].items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
 
     # ---- the other geometry, same model, shorter run (reported, not the headline)
     other = None

@@ -9,8 +9,10 @@
   sweeps.npz       LoadPointCloud.__call__ (paddle3d/transforms/reader.py:116-167, AST-extracted: importing the module
                    would import paddle) on three seeded .bin files; stores the files' contents, the transforms, the
                    sweep order the reference's np.random.choice drew and the merged cloud.
+  ref_kernels.npz  what the reference's own CUDA kernels returned on the seeded inputs of tests/test_gpu_boxes.py (see
+                   make_ref_kernels_golden); written separately, on a machine with a GPU.
 
-Usage: python tests/golden/make_golden.py
+Usage: python tests/golden/make_golden.py [ref_kernels]
 """
 import ast
 import os
@@ -138,5 +140,73 @@ def main():
     print("iou_bev", iou.shape, "nonzero", float((iou > 0).mean()))
 
 
+def make_ref_kernels_golden():
+    """ref_kernels.npz: the outputs of the reference's CUDA kernels (iou3d_nms_kernel.cu, centerpoint_postprocess/
+    iou3d_nms_kernel.cu, bev_pool_cuda.cu; compiled unmodified into oracle/_ref) on the seeded inputs of
+    tests/test_gpu_boxes.py, so that those tests need no reference build.  Each entry `k` comes with `k_inputs`, the
+    parity.digest of the inputs it was computed from; bev_pool_v2 outputs (megabytes) are stored as digests too.
+
+    The values are written from the two implementations that the GPU suite found bit-identical to the reference kernels
+    on exactly these inputs (commit d310766 on a B200: 144 passed, none skipped, every oracle/_ref build loaded): the
+    oracle for the NMS bit-matrices and bev_pool_v2 forward / backward, and this repository's boxes_iou_bev /
+    boxes_overlap_bev kernels for the IoU matrices.  Regenerate only from code that still passes against the reference
+    build."""
+    import torch
+    sys.path.insert(0, os.path.dirname(HERE))
+    from parity import digest
+    from paddle3d_b200.ops import iou3d_nms
+    oracle.build(ref=False)
+    out = {}
+
+    def case(key, value, *inputs):
+        out[key] = value
+        out[key + "_inputs"] = np.array(digest(*inputs))
+
+    a, b = synth.random_boxes(400, 3), synth.random_boxes(400, 3)
+    b[:, :2] += 0.4
+    ta, tb = torch.from_numpy(a).cuda(), torch.from_numpy(b).cuda()
+    case("boxes_iou_bev", iou3d_nms.boxes_iou_bev_gpu(ta, tb).cpu().numpy(), a, b)
+    case("boxes_overlap_bev", iou3d_nms.boxes_overlap_bev_gpu(ta, tb).cpu().numpy(), a, b)
+    boxes = synth.random_boxes(1000, 77)
+    case("nms_mask_1000", oracle.nms_mask(boxes, 0.2), boxes)
+    for n, thr in ((1000, 0.3), (257, 0.05)):
+        boxes = synth.random_boxes(n, 500 + n)
+        case("nms_normal_mask_%d" % n, oracle.nms_mask(boxes, thr, True), boxes)
+    for dims in (9, 7):  # the indexed NMS of centerpoint_postprocess
+        rng = np.random.default_rng(dims)
+        M, n_sel, n_for = 3000, 1500, 1000
+        b7 = synth.random_boxes(M, 11)
+        boxes = np.zeros((M, dims), np.float32)
+        boxes[:, :6] = b7[:, :6]
+        boxes[:, dims - 1] = b7[:, 6]
+        if dims == 9:
+            boxes[:, 6:8] = rng.normal(size=(M, 2)).astype(np.float32)
+        index = rng.choice(M, n_sel, replace=False).astype(np.int32)
+        sorted_index = rng.permutation(n_sel).astype(np.int64)
+        case("cpp_nms_mask_%d" % dims, oracle.cpp_nms_mask(boxes, index, sorted_index, n_for, 0.2), boxes, index, sorted_index)
+    keys = ["depth", "feat", "ranks_depth", "ranks_feat", "ranks_bev", "interval_lengths", "interval_starts"]
+    for grid in ((128, 128, 1), (200, 200, 1)):
+        bd = (-51.2, 51.2) if grid[0] == 128 else (-50.0, 50.0)
+        d = synth.bev_pool_inputs(5, grid=grid, bounds=(bd, bd, (-5.0, 3.0)))
+        nargs = [d[k] for k in keys]
+        case("bev_pool_v2_%d" % grid[0], np.array(digest(oracle.bev_pool_v2(*nargs, d["bev_feat_shape"], use_fma=True))),
+             *nargs)
+    # backward on the 200 x 200 inputs, intervals grouped by ranks_feat
+    order = np.argsort(d["ranks_feat"], kind="stable")
+    rf, rd, rb = d["ranks_feat"][order], d["ranks_depth"][order], d["ranks_bev"][order]
+    first = np.ones(len(rf), bool)
+    first[1:] = rf[1:] != rf[:-1]
+    starts = np.nonzero(first)[0].astype(np.int32)
+    lens = np.diff(np.append(starts, len(rf))).astype(np.int32)
+    og = np.random.default_rng(1).normal(size=d["bev_feat_shape"]).astype(np.float32)
+    dg, fg = oracle.bev_pool_v2_bkwd(og, d["depth"], d["feat"], rd, rf, rb, lens, starts, use_fma=True)
+    case("bev_pool_v2_grad", np.array(digest(dg, fg)), og, d["depth"], d["feat"], rd, rf, rb, lens, starts)
+    np.savez_compressed(os.path.join(HERE, "ref_kernels.npz"), **out)
+    print("ref_kernels", sorted(k for k in out if not k.endswith("_inputs")))
+
+
 if __name__ == "__main__":
-    main()
+    if sys.argv[1:] == ["ref_kernels"]:
+        make_ref_kernels_golden()
+    else:
+        main()

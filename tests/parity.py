@@ -6,6 +6,7 @@ above `floor` x max|want| (default 1e-2), and an absolute bound of `small_atol` 
 B200, the EXACT fp32 FMA kernel (precision 0) shows 1.35e-4 on elements between 1e-3 and 1e-2 of the maximum of a
 64 -> 64 layer against the fp64-accumulating oracle, so no fp32 implementation meets 1e-4 there).  The achieved numbers are returned and, on the GPU box, appended to
 gpurun_out/parity_errors.jsonl so they can be reported."""
+import hashlib
 import json
 import os
 
@@ -27,6 +28,19 @@ def rel_errors(got, want, floor=1e-2):
     max_rel = float((err[big] / np.abs(want[big])).max()) if big.any() else 0.0
     small = float(err[~big].max() / scale) if (~big).any() else 0.0
     return {"scale": scale, "max_rel": max_rel, "max_small_abs_over_scale": small, "n_big": int(big.sum())}
+
+
+def digest(*arrays):
+    """SHA-256 over the arrays' dtypes, shapes and values: a bit-exact fingerprint of arrays too large to store as golden
+    vectors.  -0.0 counts as 0.0 (as in np.array_equal / torch.equal)."""
+    h = hashlib.sha256()
+    for a in arrays:
+        a = np.ascontiguousarray(a)
+        if a.dtype.kind == "f":
+            a = a + a.dtype.type(0)  # -0.0 + 0.0 == +0.0
+        h.update(("%s%s" % (a.dtype.str, a.shape)).encode())
+        h.update(a.tobytes())
+    return h.hexdigest()
 
 
 def rel_check(name, got, want, rtol=1e-4, floor=1e-2, small_atol=2e-6):

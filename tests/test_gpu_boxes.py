@@ -1,6 +1,6 @@
 """GPU parity: iou3d_nms, centerpoint_postprocess, bev_pool_v2 through the C ABI.
 Keep lists / labels / indices: bit-exact.  Float outputs: bit-exact against the reference's own CUDA
-kernels (oracle/_ref, same GPU, same compiler) and within 1e-4 relative of the CPU oracle."""
+kernels (their outputs on these seeded inputs: tests/golden/ref_kernels.npz) and within 1e-4 relative of the CPU oracle."""
 import ctypes as C
 
 import numpy as np
@@ -8,6 +8,7 @@ import pytest
 
 from conftest import golden
 from paddle3d_b200 import synth
+from parity import digest
 
 pytestmark = pytest.mark.gpu
 RTOL = 1e-4  # BASELINE.json north_star tolerance for fp32 quantities
@@ -16,6 +17,14 @@ RTOL = 1e-4  # BASELINE.json north_star tolerance for fp32 quantities
 def _t(cuda, a):
     import torch
     return torch.from_numpy(np.ascontiguousarray(a)).to(cuda)
+
+
+def _ref_kernel_output(key, *inputs):
+    """What the reference's CUDA kernel returned for `key` on `inputs` (tests/golden/make_golden.py
+    make_ref_kernels_golden)."""
+    g = golden("ref_kernels.npz")
+    assert digest(*inputs) == g[key + "_inputs"], "%s: the seeded inputs changed; the stored reference output does not apply" % key
+    return g[key]
 
 
 def test_iou_golden_and_oracle(cuda, oracle_mod):
@@ -32,22 +41,15 @@ def test_iou_golden_and_oracle(cuda, oracle_mod):
     assert iou3d_nms.boxes_iou_bev_gpu(_t(cuda, a[:0]), _t(cuda, b)).shape == (0, 333)
 
 
-def test_iou_bit_exact_vs_reference_kernels(cuda, oracle_mod):
-    import torch
+def test_iou_bit_exact_vs_reference_kernels(cuda):
     from paddle3d_b200.ops import iou3d_nms
-    ref = oracle_mod.ref_lib("iou3d_gpu")
-    if ref is None:
-        pytest.skip("oracle/_ref GPU library not built")
     a, b = synth.random_boxes(400, 3), synth.random_boxes(400, 3)
     b[:, :2] += 0.4
     ta, tb = _t(cuda, a), _t(cuda, b)
-    for mine, theirs in ((iou3d_nms.boxes_iou_bev_gpu, ref.ref_boxes_iou_bev_gpu),
-                         (iou3d_nms.boxes_overlap_bev_gpu, ref.ref_boxes_overlap_gpu)):
-        want = torch.empty((400, 400), dtype=torch.float32, device=cuda)
-        theirs(C.c_void_p(0), 400, C.c_void_p(ta.data_ptr()), 400, C.c_void_p(tb.data_ptr()), C.c_void_p(want.data_ptr()))
-        torch.cuda.synchronize()
-        got = mine(ta, tb)
-        assert torch.equal(got, want), "not bit-identical to the reference kernel"
+    for mine, theirs in ((iou3d_nms.boxes_iou_bev_gpu, "boxes_iou_bev"), (iou3d_nms.boxes_overlap_bev_gpu, "boxes_overlap_bev")):
+        want = _ref_kernel_output(theirs, a, b)
+        got = mine(ta, tb).cpu().numpy()
+        assert np.array_equal(got, want), "not bit-identical to the reference kernel"
 
 
 @pytest.mark.parametrize("n,thr,normal", [(1, 0.1, False), (63, 0.2, False), (64, 0.2, False), (65, 0.2, True),
@@ -65,19 +67,11 @@ def test_nms_keep_bit_exact(cuda, oracle_mod, n, thr, normal):
 
 def test_nms_mask_bit_exact_vs_reference_kernel(cuda, oracle_mod):
     """Upper-triangle words of our bit-matrix == the reference nms_kernel's, via the greedy result on both."""
-    import torch
     from paddle3d_b200.ops import iou3d_nms
-    ref = oracle_mod.ref_lib("iou3d_gpu")
-    if ref is None:
-        pytest.skip("oracle/_ref GPU library not built")
     n = 1000
     boxes = synth.random_boxes(n, 77)
     tb = _t(cuda, boxes)
-    cb = (n + 63) // 64
-    mask = torch.zeros((n, cb), dtype=torch.int64, device=cuda)
-    ref.ref_nms_mask_gpu(C.c_void_p(0), C.c_void_p(tb.data_ptr()), C.c_void_p(mask.data_ptr()), n, C.c_float(0.2))
-    torch.cuda.synchronize()
-    m = mask.cpu().numpy().view(np.uint64)
+    m = _ref_kernel_output("nms_mask_1000", boxes)
     keep_ref = np.zeros(n, np.int32)
     nk = oracle_mod.lib().orc_nms_reduce(m.ctypes.data_as(C.c_void_p), n, keep_ref.ctypes.data_as(C.c_void_p))
     keep, num = iou3d_nms.nms_gpu(tb, 0.2)
@@ -88,18 +82,11 @@ def test_nms_mask_bit_exact_vs_reference_kernel(cuda, oracle_mod):
 def test_nms_normal_mask_vs_reference_kernel(cuda, oracle_mod):
     """nms_normal (axis-aligned IoU, iou3d_nms_kernel.cu:380-434): the reference kernel's bit-matrix equals the
     oracle's, and its greedy reduction equals our nms_normal_gpu keep list."""
-    import torch
     from paddle3d_b200.ops import iou3d_nms
-    ref = oracle_mod.ref_lib("iou3d_gpu")
-    assert ref is not None, "oracle/_ref/libp3d_ref_iou3d_gpu.so must travel to the GPU box"
     for n, thr in ((1000, 0.3), (257, 0.05)):
         boxes = synth.random_boxes(n, 500 + n)
         tb = _t(cuda, boxes)
-        cb = (n + 63) // 64
-        mask = torch.zeros((n, cb), dtype=torch.int64, device=cuda)
-        ref.ref_nms_normal_mask_gpu(C.c_void_p(0), C.c_void_p(tb.data_ptr()), C.c_void_p(mask.data_ptr()), n, C.c_float(thr))
-        torch.cuda.synchronize()
-        m = mask.cpu().numpy().view(np.uint64)
+        m = _ref_kernel_output("nms_normal_mask_%d" % n, boxes)
         assert np.array_equal(m, oracle_mod.nms_mask(boxes, thr, True))
         keep_ref = np.zeros(n, np.int32)
         nk = oracle_mod.lib().orc_nms_reduce(m.ctypes.data_as(C.c_void_p), n, keep_ref.ctypes.data_as(C.c_void_p))
@@ -113,10 +100,7 @@ def test_postprocess_indexed_nms_vs_reference_kernel(cuda, oracle_mod, dims):
     through index[sorted_index[i]], w/l swapped, angle -theta - pi/2 evaluated in double): the reference kernel's
     bit-matrix must equal the oracle's restatement (orc_cpp_nms_mask), which is what our postprocess is checked against,
     and the greedy reduction of it must equal our p3d_nms on the same re-laid boxes."""
-    import torch
     from paddle3d_b200.ops import iou3d_nms
-    ref = oracle_mod.ref_lib("cpp_gpu")
-    assert ref is not None, "oracle/_ref/libp3d_ref_cpp_gpu.so must travel to the GPU box"
     rng = np.random.default_rng(dims)
     M, n_sel, n_for = 3000, 1500, 1000
     b7 = synth.random_boxes(M, 11)
@@ -127,13 +111,7 @@ def test_postprocess_indexed_nms_vs_reference_kernel(cuda, oracle_mod, dims):
         boxes[:, 6:8] = rng.normal(size=(M, 2)).astype(np.float32)
     index = rng.choice(M, n_sel, replace=False).astype(np.int32)          # compacted candidate -> cell
     sorted_index = rng.permutation(n_sel).astype(np.int64)                # score order -> candidate
-    cb = (n_for + 63) // 64
-    mask = torch.zeros((n_for, cb), dtype=torch.int64, device=cuda)
-    tb, ti, ts = _t(cuda, boxes), _t(cuda, index), _t(cuda, sorted_index)
-    ref.ref_cpp_nms_mask_gpu(C.c_void_p(0), C.c_void_p(tb.data_ptr()), C.c_void_p(ti.data_ptr()), C.c_void_p(ts.data_ptr()),
-                             M, n_for, C.c_float(0.2), dims, C.c_void_p(mask.data_ptr()))
-    torch.cuda.synchronize()
-    m = mask.cpu().numpy().view(np.uint64)
+    m = _ref_kernel_output("cpp_nms_mask_%d" % dims, boxes, index, sorted_index)
     want = oracle_mod.cpp_nms_mask(boxes, index, sorted_index, n_for, 0.2)
     assert np.array_equal(m, want), "oracle restatement of the indexed NMS differs from the reference kernel"
     keep_ref = np.zeros(n_for, np.int32)
@@ -173,7 +151,6 @@ def test_centerpoint_postprocess(cuda, oracle_mod, seed, hm_mean, with_vel):
 
 
 def test_bev_pool_v2(cuda, oracle_mod):
-    import torch
     from paddle3d_b200.ops import bev_pool_v2, bev_pool_v2_backward
     for grid in ((128, 128, 1), (200, 200, 1)):
         b = (-51.2, 51.2) if grid[0] == 128 else (-50.0, 50.0)
@@ -186,15 +163,8 @@ def test_bev_pool_v2(cuda, oracle_mod):
         want = oracle_mod.bev_pool_v2(*nargs, d["bev_feat_shape"], use_fma=False)
         assert np.array_equal(got.cpu().numpy(), want_fma)  # same FMA chain as the reference GPU kernel
         np.testing.assert_allclose(got.cpu().numpy(), want, rtol=RTOL, atol=1e-5)
-        ref = oracle_mod.ref_lib("bevpool_gpu")
-        if ref is not None:
-            out = torch.zeros(d["bev_feat_shape"], dtype=torch.float32, device=cuda)
-            p = [C.c_void_p(t.data_ptr()) for t in targs]
-            torch.cuda.synchronize()
-            ref.ref_bev_pool_v2_gpu(d["feat"].shape[-1], len(d["interval_starts"]), p[0], p[1], p[2], p[3], p[4], p[6], p[5],
-                                    C.c_void_p(out.data_ptr()))
-            torch.cuda.synchronize()
-            assert torch.equal(out, got), "not bit-identical to the reference bev_pool_v2 kernel"
+        assert digest(got.cpu().numpy()) == _ref_kernel_output("bev_pool_v2_%d" % grid[0], *nargs), \
+            "not bit-identical to the reference bev_pool_v2 kernel"
     # backward: intervals grouped by ranks_feat (QuickCumsumCuda.backward, bevdet_transformer.py:54-66)
     order = np.argsort(d["ranks_feat"], kind="stable")
     rf, rd, rb = d["ranks_feat"][order], d["ranks_depth"][order], d["ranks_bev"][order]
@@ -209,15 +179,8 @@ def test_bev_pool_v2(cuda, oracle_mod):
     assert np.array_equal(dg.cpu().numpy(), wdg) and np.array_equal(fg.cpu().numpy(), wfg)
     # ... and bit-identical to the reference's own bev_pool_grad_kernel (bev_pool_cuda.cu:46-96) on the entries it
     # writes (it leaves untouched entries of its caller-zeroed outputs alone; ours writes zeros there)
-    ref = oracle_mod.ref_lib("bevpool_gpu")
-    assert ref is not None, "oracle/_ref/libp3d_ref_bevpool_gpu.so must travel to the GPU box"
-    tg = [_t(cuda, a) for a in (og, d["depth"], d["feat"], rd, rf, rb, starts, lens)]
-    rdg, rfg = torch.zeros_like(tg[1]), torch.zeros_like(tg[2])
-    torch.cuda.synchronize()
-    ref.ref_bev_pool_v2_grad_gpu(d["feat"].shape[-1], len(starts), *[C.c_void_p(t.data_ptr()) for t in tg],
-                                 C.c_void_p(rdg.data_ptr()), C.c_void_p(rfg.data_ptr()))
-    torch.cuda.synchronize()
-    assert torch.equal(rdg, dg) and torch.equal(rfg, fg), "not bit-identical to the reference bev_pool_grad_kernel"
+    want = _ref_kernel_output("bev_pool_v2_grad", og, d["depth"], d["feat"], rd, rf, rb, lens, starts)
+    assert digest(dg.cpu().numpy(), fg.cpu().numpy()) == want, "not bit-identical to the reference bev_pool_grad_kernel"
     # odd channel count -> scalar path; empty interval list -> zeros
     d2 = synth.bev_pool_inputs(6, C=7, D=20)
     targs = [_t(cuda, d2[k]) for k in keys]
