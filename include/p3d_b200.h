@@ -391,6 +391,18 @@ int p3d_pillar_feature_net(const float *voxels, const int32_t *num_points_per_vo
                            int out_channels, const float *weight, const float *bn_scale, const float *bn_shift,
                            const float *voxel_size_host, const float *point_cloud_range_host, float *out,
                            p3d_stream_t stream);
+/* The same layer with PointPillarsScatter and the pixel fp16-pair conversion folded into its epilogue: zeroes the pixel
+ * H16 image out_pixel_h16 [batch * ny * nx][C / 32][hi 32 | lo' 32] halfs, then writes each pillar's C channels into the
+ * pixel (b * ny + y) * nx + x of its coors (b, z, y, x); z is ignored, rows outside the grid or with b >= batch are
+ * skipped.  Cells are unique by construction (hard_voxelize emits one row per cell), so there is no duplicate handling.
+ * Same fp32 arithmetic as p3d_pillar_feature_net: the image equals p3d_nchw_to_pixel_h16 of the scattered canvas bit for
+ * bit.  |x| > 65504 is saturated and sets bit 0 of *status_dev (may be NULL).  Null pointers or misaligned coors / image
+ * (16 bytes) return P3D_ERR_INVALID_ARG; max_points > 64, num_point_dim > 8 or C % 32 != 0 P3D_ERR_UNSUPPORTED. */
+int p3d_pillar_feature_net_pixel_h16(const float *voxels, const int32_t *num_points_per_voxel, const int32_t *coors,
+                                     const int32_t *num_voxels_dev, int64_t n_cap, int max_points, int num_point_dim,
+                                     int out_channels, const float *weight, const float *bn_scale, const float *bn_shift,
+                                     const float *voxel_size_host, const float *point_cloud_range_host, int batch, int ny,
+                                     int nx, void *out_pixel_h16, int32_t *status_dev, p3d_stream_t stream);
 
 #ifdef __cplusplus
 }

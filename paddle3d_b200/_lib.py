@@ -76,6 +76,8 @@ SIGNATURES = {
     "p3d_nchw_to_pixel_split": (_int, [_vp, _int, _int, _int, _int, _vp, _vp]),
     "p3d_dense_conv2d_packed_weight_bytes": (_sz, [_int, _int, _int, _int]),
     "p3d_pillar_feature_net": (_int, [_vp, _vp, _vp, _vp, _i64, _int, _int, _int, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "p3d_pillar_feature_net_pixel_h16": (_int, [_vp, _vp, _vp, _vp, _i64, _int, _int, _int, _vp, _vp, _vp, _vp, _vp, _int,
+                                                _int, _int, _vp, _vp, _vp]),
     "p3d_head_final_conv": (_int, [_vp, _int, _int, _int, _int, _int, _int, _vp, _vp, _vp, _vp, _int, _vp, _vp]),
     "p3d_head_final_conv_h16": (_int, [_vp, _int, _int, _int, _int, _int, _int, _vp, _vp, _vp, _vp, _int, _vp, _vp]),
     "p3d_nchw_to_pixel_h16": (_int, [_vp, _int, _int, _int, _int, _vp, _vp, _vp]),

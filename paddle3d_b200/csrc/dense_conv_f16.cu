@@ -24,6 +24,7 @@
 #include <cuda.h>
 #include <cuda_fp16.h>
 
+#include "h16.cuh"
 #include "p3d_b200.h"
 #include "tc_common.cuh"
 
@@ -35,7 +36,6 @@ using namespace tc;
 constexpr int kTW = 8, kTH = 16;        // output tile of one M = 128 UMMA: 8 x 16 pixels
 constexpr int kThreadsD = 7 * 32;
 constexpr int kMaxB = 12;               // weight ring depth limit
-constexpr float kLoScale = 2048.0f, kLoInv = 1.0f / 2048.0f;
 
 struct Params {
   int B, H, W, Cin;           // input image (pixel H16 rows [B*H*W][4 * Cin bytes])
@@ -131,15 +131,6 @@ __device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&a)[16]) {
         "=r"(a[9]), "=r"(a[10]), "=r"(a[11]), "=r"(a[12]), "=r"(a[13]), "=r"(a[14]), "=r"(a[15])
       : "r"(taddr));
 }
-__device__ __forceinline__ void split_h16(float x, __half &hi, __half &lo, bool &ovf) {
-  if (fabsf(x) > 65504.0f) {
-    ovf = true;
-    x = copysignf(65504.0f, x);
-  }
-  hi = __float2half_rn(x);
-  lo = __float2half_rn((x - __half2float(hi)) * kLoScale);
-}
-
 struct Item {
   int nt, tap0, tx0, ty0, b;
 };

@@ -31,6 +31,7 @@
 #include <cuda.h>
 #include <cuda_fp16.h>
 
+#include "h16.cuh"
 #include "tc_common.cuh"
 
 namespace p3d {
@@ -43,7 +44,6 @@ using namespace tc;
 constexpr int kSub = 128 * 128;  // bytes of one A sub-tile
 constexpr int kMaxSplits = 4;
 constexpr int kMaxStages = 12;
-constexpr float kLoScale = 2048.0f, kLoInv = 1.0f / 2048.0f;
 
 template <int CIN, int COUT, int NSUB_>
 struct Cfg {
@@ -112,16 +112,6 @@ __device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&a)[16]) {
 }
 __device__ __forceinline__ void epi_bar() { asm volatile("bar.sync 1, 128;" ::: "memory"); }
 
-// x -> (hi, lo') fp16 pair; sets ovf when |x| leaves fp16's range (value saturated)
-__device__ __forceinline__ void split_h16(float x, __half &hi, __half &lo, bool &ovf) {
-  if (fabsf(x) > 65504.0f) {
-    ovf = true;
-    x = copysignf(65504.0f, x);
-  }
-  hi = __float2half_rn(x);
-  lo = __float2half_rn((x - __half2float(hi)) * kLoScale);
-}
-__device__ __forceinline__ float merge_h16(__half hi, __half lo) { return fmaf(__half2float(lo), kLoInv, __half2float(hi)); }
 
 // Number of tap splits for `n_tiles` row tiles on `grid` persistent CTAs: minimise waves x (taps per item + fixed cost).
 __host__ __device__ inline int choose_splits(long long n_tiles, int grid, int K, int smax) {

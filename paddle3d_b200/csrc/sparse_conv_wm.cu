@@ -30,11 +30,11 @@
 #include <stdlib.h>
 
 #include "common.cuh"
+#include "h16.cuh"
 
 namespace p3d {
 namespace wm {
 
-constexpr float kLoScale = 2048.0f, kLoInv = 1.0f / 2048.0f;
 constexpr int kWarps = 16;  // warps per CTA of every instantiation, one CTA per SM
 
 struct Params {
@@ -60,15 +60,6 @@ __device__ __forceinline__ void mma16816(float (&c)[4], const uint4 &a, uint32_t
       : "r"(a.x), "r"(a.y), "r"(a.z), "r"(a.w), "r"(b0), "r"(b1));
 }
 
-__device__ __forceinline__ void split_h16(float x, __half &hi, __half &lo, bool &ovf) {
-  if (fabsf(x) > 65504.0f) {
-    ovf = true;
-    x = copysignf(65504.0f, x);
-  }
-  hi = __float2half_rn(x);
-  lo = __float2half_rn((x - __half2float(hi)) * kLoScale);
-}
-__device__ __forceinline__ float merge_h16(__half hi, __half lo) { return fmaf(__half2float(lo), kLoInv, __half2float(hi)); }
 
 // B-fragment words of one (tile, tap) unit for the two rows (g, g + 8) a lane serves: [row][half: hi, lo'][CIN / 8 words];
 // words 2s, 2s + 1 are (b0, b1) of k-step s

@@ -100,8 +100,15 @@ class DenseRPNHead:
             cin = cout
         self.deblocks = []
         for ci, co, u in zip(out_channels, fpn_out_channels, upsample_strides):
-            # use_conv_for_no_stride: stride 1 -> Conv2D k = 1; stride > 1 -> Conv2DTranspose k = s (second_fpn.py:118-139)
-            self.deblocks.append(conv(ci, co, 1, 1, 0, bn_eps=bn3) if u == 1 else conv(ci, co, u, u, 0, bn_eps=bn3, up=u))
+            # use_conv_for_no_stride: stride 1 -> Conv2D k = 1; stride > 1 -> Conv2DTranspose k = s; stride < 1 -> Conv2D
+            # k = s = round(1 / stride), a down-sampling deblock (second_fpn.py:118-139)
+            if u == 1:
+                self.deblocks.append(conv(ci, co, 1, 1, 0, bn_eps=bn3))
+            elif u > 1:
+                self.deblocks.append(conv(ci, co, int(u), int(u), 0, bn_eps=bn3, up=int(u)))
+            else:
+                k = int(round(1.0 / u))
+                self.deblocks.append(conv(ci, co, k, k, 0, bn_eps=bn3))
         self.fpn_channels = int(sum(fpn_out_channels))
         self.shared = conv(self.fpn_channels, share_conv_channel, 3, 1, 1, bias=True, bn_eps=bn5)
         self.heads = []  # per task: list of (name, ConvModule 64->64, final conv 64->classes)
@@ -150,6 +157,21 @@ class DenseRPNHead:
         return dict(blocks=[[c.np for c in blk] for blk in self.blocks], deblocks=[c.np for c in self.deblocks],
                     shared=self.shared.np, heads=[[(n, a.np, b.np) for n, a, b in hs] for hs in self.heads])
 
+    @staticmethod
+    def deblock_out_hw(de, h, w):
+        """Output size of a SecondFPN deblock on an h x w input: transposed conv (up > 1) or strided conv."""
+        if de.up > 1:
+            return h * de.up, w * de.up
+        return (h + 2 * de.padding - de.k) // de.stride + 1, (w + 2 * de.padding - de.k) // de.stride + 1
+
+    def fpn_out_hw(self, feat_shapes):
+        """(H, W) of the SecondFPN concat for backbone outputs of shapes (B, H, W, C); raises ValueError when the
+        deblocks bring the levels to different sizes."""
+        sizes = [self.deblock_out_hw(de, fs[1], fs[2]) for fs, de in zip(feat_shapes, self.deblocks)]
+        if len(set(sizes)) != 1:
+            raise ValueError("SecondFPN deblocks produce different sizes %s: they cannot be concatenated" % sizes)
+        return sizes[0]
+
     # ---- RPN + neck + shared conv: bev [B, C, H, W] fp32 -> (pixel rows of the shared feature map, its shape)
     def _trunk(self, bev, shape=None):
         """bev: fp32 NCHW tensor, or (shape given) pixel fp16-pair rows [B*H*W, 2*C] with shape = (B, H, W, C)."""
@@ -172,12 +194,11 @@ class DenseRPNHead:
                 x, _, (b_, oh, ow) = conv(x, shape)
                 shape = (b_, oh, ow, conv.cout)
             feats.append((x, shape))
-        cat, c0, out_hw = None, 0, None
+        out_hw = self.fpn_out_hw([fs for _, fs in feats])
+        cat = torch.empty((b * out_hw[0] * out_hw[1], 2 * self.fpn_channels),
+                          dtype=torch.float16 if self.f16 else torch.float32, device=bev.device)
+        c0 = 0
         for (f, fshape), de in zip(feats, self.deblocks):
-            if cat is None:
-                out_hw = (fshape[1] * de.up, fshape[2] * de.up)
-                cat = torch.empty((fshape[0] * out_hw[0] * out_hw[1], 2 * self.fpn_channels),
-                                  dtype=torch.float16 if self.f16 else torch.float32, device=bev.device)
             de(f, fshape, out_split=cat, out_channels=self.fpn_channels, out_c0=c0)
             c0 += de.cout
         H, W = out_hw

@@ -2,6 +2,7 @@
 
     HardVoxelizer        paddle3d/models/voxelizers/voxelize.py:26-82
     VoxelMean            paddle3d/models/voxel_encoders/voxel_encoder.py:42-57
+    PillarFeatureNet     paddle3d/models/voxel_encoders/pillar_encoder.py:115-210
     PointPillarsScatter  paddle3d/models/middle_encoders/pillar_scatter.py:27-105
     SparseResNet3D       paddle3d/models/middle_encoders/sparse_resnet.py:114-206
     SparseNet3D          paddle3d/models/middle_encoders/sparsenet.py:67-182 (PV-RCNN / Voxel-RCNN family)
@@ -96,6 +97,58 @@ class PointPillarsScatter:
     def forward(self, voxel_features, coords, batch_size, num=None):
         """[n, C] + [n, 4] (b, z, y, x) -> [batch, C, ny, nx]."""
         return _ps.pillar_scatter(voxel_features, coords, batch_size, self.ny, self.nx, num)
+
+    __call__ = forward
+
+
+class PillarFeatureNet:
+    """PillarFeatureNet (voxel_encoders/pillar_encoder.py:115-210) with its one PFNLayer (Linear without bias,
+    BatchNorm1D eps 1e-3, ReLU, max over the points of a pillar) as one launch.  Decoration: the point features, xyz minus
+    the pillar's mean and xy minus the pillar's centre (F + 5 inputs).  `legacy` only changes the reference's training-time
+    layer layout, not this inference arithmetic; several PFN layers and `with_distance` are not implemented."""
+
+    def __init__(self, in_channels=4, feat_channels=(64,), with_distance=False, max_num_points_in_voxel=100,
+                 voxel_size=(0.2, 0.2, 4), point_cloud_range=(0, -40, -3, 70.4, 40, 1), legacy=True):
+        feat_channels = list(feat_channels)
+        if len(feat_channels) != 1:
+            raise ValueError("PillarFeatureNet: exactly one PFN layer is supported, got feat_channels=%s" % feat_channels)
+        if with_distance:
+            raise ValueError("PillarFeatureNet: with_distance=True is not supported")
+        self.in_channels, self.out_channels = int(in_channels), int(feat_channels[0])
+        self.max_num_points_in_voxel, self.legacy = int(max_num_points_in_voxel), legacy
+        self.voxel_size = list(map(float, voxel_size))
+        self.point_cloud_range = list(map(float, point_cloud_range))
+        self.np = None
+        self.weight = self.folded = None
+
+    def init_weight(self, seed=0, device="cuda", bn_gain=1.0):
+        """Seeded Linear weight [F + 5, C] (kaiming-uniform bound, as synth.kaiming_uniform) and BatchNorm1D with
+        gamma = bn_gain, beta 0, mean 0, var 1; folded into (scale, shift) once.  device=None: numpy parameters only."""
+        rng = np.random.default_rng(seed)
+        d, c = self.in_channels + 5, self.out_channels
+        from .synth import kaiming_uniform
+        self.np = dict(weight=kaiming_uniform(rng, (d, c), d), gamma=np.full(c, bn_gain, np.float32),
+                       beta=np.zeros(c, np.float32), mean=np.zeros(c, np.float32), var=np.ones(c, np.float32), eps=1e-3)
+        if device is not None:
+            from .ops.pillar_encoder import fold_bn
+            p = self.np
+            self.weight = torch.from_numpy(p["weight"]).to(device)
+            self.folded = fold_bn(p["gamma"], p["beta"], p["mean"], p["var"], p["eps"], device)
+        return self
+
+    def forward(self, features, num_points_per_voxel, coors, num=None):
+        """features [n, M, F], counts [n], coors [n, 4] (b, z, y, x) -> pillar features [n, C]."""
+        from .ops.pillar_encoder import pillar_feature_net
+        return pillar_feature_net(features, num_points_per_voxel, coors, self.weight, None, None, None, None, None,
+                                  self.voxel_size, self.point_cloud_range, num_voxels=num, folded=self.folded)
+
+    def forward_pixel_h16(self, features, num_points_per_voxel, coors, batch, ny, nx, num=None):
+        """Same features, scattered straight into the pixel fp16-pair image: (rows [batch * ny * nx, 2 * C] float16,
+        (batch, ny, nx, C)), the input of DenseRPNHead.forward_h16."""
+        from .ops.pillar_encoder import pillar_feature_net_pixel_h16
+        return pillar_feature_net_pixel_h16(features, num_points_per_voxel, coors, self.weight, None, None, None, None, None,
+                                            self.voxel_size, self.point_cloud_range, batch, ny, nx, num_voxels=num,
+                                            folded=self.folded)
 
     __call__ = forward
 

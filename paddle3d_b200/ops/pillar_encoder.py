@@ -34,3 +34,29 @@ def pillar_feature_net(voxels, num_points_per_voxel, coors, weight, bn_gamma, bn
                                        ptr(shift), host_floats(voxel_size), host_floats(point_cloud_range), ptr(out),
                                        stream(dev)), "pillar_feature_net")
     return out
+
+
+def pillar_feature_net_pixel_h16(voxels, num_points_per_voxel, coors, weight, bn_gamma, bn_beta, bn_mean, bn_var, bn_eps,
+                                 voxel_size, point_cloud_range, batch, ny, nx, num_voxels=None, folded=None):
+    """pillar_feature_net + PointPillarsScatter + nchw_to_pixel_h16 in one launch (after a zero fill of the image):
+    returns (image [batch * ny * nx, 2 * C] float16 pixel fp16-pair rows, (batch, ny, nx, C)), the input of
+    DenseRPNHead.forward_h16.  Values above fp16's range are saturated and set bit 0 of sparse_nn.status_tensor."""
+    from .sparse_nn import status_tensor
+    voxels = require_cuda(voxels, "voxels", torch.float32)
+    npv = require_cuda(num_points_per_voxel, "num_points_per_voxel", torch.int32)
+    coors = require_cuda(coors, "coors", torch.int32)
+    weight = require_cuda(weight, "weight", torch.float32)
+    n, m, f = voxels.shape
+    c = weight.shape[1]
+    if weight.shape[0] != f + 5:
+        raise ValueError("weight must be [F + 5, C]")
+    dev = voxels.device
+    scale, shift = folded if folded is not None else fold_bn(bn_gamma, bn_beta, bn_mean, bn_var, bn_eps, dev)
+    batch, ny, nx = int(batch), int(ny), int(nx)
+    out = torch.empty((batch * ny * nx, 2 * c), dtype=torch.float16, device=dev)
+    nump = ptr(require_cuda(num_voxels, "num_voxels", torch.int32)) if num_voxels is not None else ptr(None)
+    check(lib().p3d_pillar_feature_net_pixel_h16(ptr(voxels), ptr(npv), ptr(coors), nump, n, m, f, c, ptr(weight),
+                                                 ptr(scale), ptr(shift), host_floats(voxel_size),
+                                                 host_floats(point_cloud_range), batch, ny, nx, ptr(out),
+                                                 ptr(status_tensor(dev)), stream(dev)), "pillar_feature_net_pixel_h16")
+    return out, (batch, ny, nx, c)

@@ -1,4 +1,7 @@
-"""CenterPoint-voxel hot-path frame on one B200: the public API a user calls (bench.py `e2e`).
+"""CenterPoint hot-path frames on one B200: the public API a user calls (bench.py `e2e`).  CenterPointHotPath is the voxel
+model (below); CenterPointPillarsHotPath the 0.2 m pillar model (hard_voxelize -> PillarFeatureNet into the pixel fp16-pair
+BEV image -> the same dense RPN / neck / CenterHead -> centerpoint_postprocess).  Both share their frame I/O
+(_FramePipeline) and run side by side in CenterPointSweep lanes.
 
     voxelize (+ VoxelMean fused)  ->  SparseResNet3D (21 sparse convs)  ->  dense BEV [1,256,180,180]
     -> dense 2-D RPN + neck + CenterHead (with_head=True; otherwise resident synthetic head tensors)
@@ -18,6 +21,10 @@ from .layers import SparseResNet3D
 from .ops import centerpoint_postprocess as cpp
 from .ops import sparse_nn as sp
 from .ops import voxelize as vox
+
+# BatchNorm gamma of the seeded pillar model (PillarFeatureNet and dense head): keeps the activations O(1) through the
+# 1 + 16 + 3 + 1 + 36 layers of the frame (see DESIGN.md §1)
+PILLARS_BN_GAIN = 6.0 ** 0.5
 
 
 def _count_graph_nodes(raw_graph):
@@ -40,32 +47,14 @@ def _count_graph_nodes(raw_graph):
     return out
 
 
-class CenterPointHotPath:
-    def __init__(self, cfg=None, device="cuda:0", precision=sp.FP32, seed=0, num_points=None, level_caps=None,
-                 head_seed=0, with_head=False, keep_bev=True, bn_gain=1.0):
-        self.cfg = dict(cfg or synth.C3)
-        self.device = torch.device(device)
-        self.n = int(num_points or self.cfg["num_points"])
-        self.F = self.cfg["point_dim"]
-        self.test_cfg = dict(synth.CENTERPOINT_TEST_CFG)
-        self.label_off = synth.label_offsets()
-        self.net = SparseResNet3D(self.F, self.cfg["voxel_size"], self.cfg["point_cloud_range"])
-        self.net.init_weight(seed=seed, device=self.device, bn_gain=bn_gain).set_precision(precision)
-        V = self.cfg["max_voxels"]
-        self.net.set_level_caps(level_caps or [3 * V, 3 * V, 2 * V, V])
-        h = synth.centerpoint_head_outputs(head_seed)
-        self.head_host = h
-        self.head = {k: [torch.from_numpy(x).to(self.device) for x in v] for k, v in h.items()}
-        # with_head: run the dense RPN / neck / CenterHead (dense_head.DenseRPNHead, SURVEY §8f-1) on the BEV tensor and
-        # feed ITS outputs to the postprocess instead of the resident synthetic head tensors (parity-green per layer and
-        # as a small network; this whole-frame composition has not been timed yet, hence off by default)
-        self.dense = None
-        if with_head:
-            from .dense_head import DenseRPNHead
-            self.dense = DenseRPNHead(in_channels=128 * 2).init_weight(seed=seed + 1, device=self.device, bn_gain=bn_gain)
-        # keep_bev=False (with the fp16-pair dense head): the sparse rows go straight into the pixel fp16-pair image the RPN
-        # reads; the reference's fp32 NCHW BEV tensor is then not materialised in the frame (bev_nchw() rebuilds it on demand)
-        self.keep_bev = keep_bev or self.dense is None or not self.dense.f16
+class _FramePipeline:
+    """Frame I/O shared by the CenterPoint pipelines: the static device input, the pipeline stream, the CUDA graph of
+    one frame and the pinned result buffers; infer / infer_many / capture / launch around the subclass's
+    forward_device() (one frame enqueued on the current stream, returning a dict with at least boxes, scores, labels,
+    counts and status) and check_status() (raises on a non-zero device status word)."""
+
+    def _init_io(self, status_words):
+        """Needs self.n, self.F, self.device, self.label_off and self.test_cfg."""
         self.points = torch.zeros((self.n, self.F), dtype=torch.float32, device=self.device)  # static input
         self.graph = None
         self.out = None
@@ -75,61 +64,7 @@ class CenterPointHotPath:
         self.h_scores = torch.empty((rows,), dtype=torch.float32).pin_memory()
         self.h_labels = torch.empty((rows,), dtype=torch.int64).pin_memory()
         self.h_counts = torch.empty((len(self.label_off) + 1,), dtype=torch.int32).pin_memory()
-        self.h_status = torch.zeros((5,), dtype=torch.int32).pin_memory()
-
-    # ---- one frame, enqueued on the current stream, device in / device out
-    def forward_device(self):
-        cfg, tc = self.cfg, self.test_cfg
-        mean, coors, npv, nv = vox.voxelize_mean(self.points, cfg["voxel_size"], cfg["point_cloud_range"],
-                                                 cfg["max_points"], cfg["max_voxels"], 0)
-        bev, bev_h16 = None, None
-        if self.keep_bev:
-            bev = self.net(mean, coors, 1, num=nv)
-            h = self.dense(bev) if self.dense is not None else self.head
-        else:
-            bev_h16 = self.net(mean, coors, 1, num=nv, pixel_h16=True)
-            h = self.dense.forward_h16(*bev_h16)
-        # frame status word (ADVICE r1): [fp16-range overflow of the pair-row kernels, overflow flag of each strided level]
-        status = torch.stack([sp.status_tensor(self.device)[0]] + [c[1] for c in self.net.level_counters])
-        boxes, scores, labels, counts = cpp.centerpoint_postprocess_device(
-            h["hm"], h["reg"], h["height"], h["dim"], h["vel"], h["rot"], cfg["voxel_size"][:2],
-            cfg["point_cloud_range"], tc["post_center_limit_range"], self.label_off, tc["down_ratio"],
-            tc["score_threshold"], tc["nms_iou_threshold"], tc["nms_pre_max_size"], tc["nms_post_max_size"], True)
-        return dict(bev=bev, bev_h16=bev_h16, boxes=boxes, scores=scores, labels=labels, counts=counts, num_voxels=nv,
-                    coors=coors, mean=mean, status=status)
-
-    def bev_nchw(self):
-        """The dense BEV tensor [1, 256, H, W] fp32 of the last frame (rebuilt from the pixel fp16-pair image when the
-        frame did not materialise it)."""
-        if self.out["bev"] is not None:
-            self.stream.synchronize()
-            return self.out["bev"]
-        from .ops import dense_conv as dc
-        rows, shape = self.out["bev_h16"]
-        with torch.cuda.stream(self.stream):
-            out = dc.pixel_h16_to_nchw(rows, shape)
-            # pixel rows hold (z, c)-ordered channels (to_pixel_h16); the reference tensor is (c, z)-ordered
-            b, h, w, cd = shape
-            D = self.dense.bev_depth
-            out = out.view(b, D, cd // D, h, w).transpose(1, 2).reshape(b, cd, h, w).contiguous()
-        self.stream.synchronize()  # callers read it from other streams
-        return out
-
-    def calibrate_head(self, points_dev):
-        """Shift the heat-map biases of the (randomly initialised) dense head so that ~1.4 % of the BEV cells of this frame
-        score above the threshold, as SURVEY.md §8d specifies for the synthetic workload (see
-        DenseRPNHead.calibrate_heatmap_bias).  Call before capture()."""
-        if self.dense is None:
-            return self
-        cfg = self.cfg
-        with torch.cuda.stream(self.stream):
-            self.points.copy_(points_dev)
-            mean, coors, npv, nv = vox.voxelize_mean(self.points, cfg["voxel_size"], cfg["point_cloud_range"],
-                                                     cfg["max_points"], cfg["max_voxels"], 0)
-            bev = self.net(mean, coors, 1, num=nv)
-            self.dense.calibrate_heatmap_bias(bev, self.test_cfg["score_threshold"])
-        self.stream.synchronize()
-        return self
+        self.h_status = torch.zeros((status_words,), dtype=torch.int32).pin_memory()
 
     def capture(self, warmup=2, count_nodes=False):
         """Warm up (sizes the workspaces) on the side stream, then capture the frame into a CUDA graph.  count_nodes:
@@ -175,18 +110,6 @@ class CenterPointHotPath:
         self.check_status(self.h_status)
         k = int(self.h_counts[-1])
         return self.h_boxes[:k], self.h_scores[:k], self.h_labels[:k]
-
-    @staticmethod
-    def check_status(status_host):
-        """Raise when the frame's device status word reports dropped work (never a silent wrong result)."""
-        st = [int(v) for v in status_host]
-        if st[0]:
-            raise RuntimeError("sparse backbone: an activation left fp16's range (|x| >= 65504) on the fp16-pair path; "
-                               "run this model with precision TF32X3_SPLIT")
-        for lvl, v in enumerate(st[1:]):
-            if v:
-                raise RuntimeError("sparse backbone: strided level %d overflowed its row capacity (set_level_caps); "
-                                   "output sites were dropped" % (lvl + 1))
 
     # ---- public end-to-end call for a sweep of frames: same per-frame work, copies overlapped with compute
     def prepare_sweep(self):
@@ -257,6 +180,101 @@ class CenterPointHotPath:
                self.h_status.numel() * 4)
         return h2d, d2h
 
+
+class CenterPointHotPath(_FramePipeline):
+    def __init__(self, cfg=None, device="cuda:0", precision=sp.FP32, seed=0, num_points=None, level_caps=None,
+                 head_seed=0, with_head=False, keep_bev=True, bn_gain=1.0):
+        self.cfg = dict(cfg or synth.C3)
+        self.device = torch.device(device)
+        self.n = int(num_points or self.cfg["num_points"])
+        self.F = self.cfg["point_dim"]
+        self.test_cfg = dict(synth.CENTERPOINT_TEST_CFG)
+        self.label_off = synth.label_offsets()
+        self.net = SparseResNet3D(self.F, self.cfg["voxel_size"], self.cfg["point_cloud_range"])
+        self.net.init_weight(seed=seed, device=self.device, bn_gain=bn_gain).set_precision(precision)
+        V = self.cfg["max_voxels"]
+        self.net.set_level_caps(level_caps or [3 * V, 3 * V, 2 * V, V])
+        h = synth.centerpoint_head_outputs(head_seed)
+        self.head_host = h
+        self.head = {k: [torch.from_numpy(x).to(self.device) for x in v] for k, v in h.items()}
+        # with_head: run the dense RPN / neck / CenterHead (dense_head.DenseRPNHead, SURVEY §8f-1) on the BEV tensor and
+        # feed ITS outputs to the postprocess instead of the resident synthetic head tensors (parity-green per layer and
+        # as a small network; this whole-frame composition has not been timed yet, hence off by default)
+        self.dense = None
+        if with_head:
+            from .dense_head import DenseRPNHead
+            self.dense = DenseRPNHead(in_channels=128 * 2).init_weight(seed=seed + 1, device=self.device, bn_gain=bn_gain)
+        # keep_bev=False (with the fp16-pair dense head): the sparse rows go straight into the pixel fp16-pair image the RPN
+        # reads; the reference's fp32 NCHW BEV tensor is then not materialised in the frame (bev_nchw() rebuilds it on demand)
+        self.keep_bev = keep_bev or self.dense is None or not self.dense.f16
+        self._init_io(5)
+
+    # ---- one frame, enqueued on the current stream, device in / device out
+    def forward_device(self):
+        cfg, tc = self.cfg, self.test_cfg
+        mean, coors, npv, nv = vox.voxelize_mean(self.points, cfg["voxel_size"], cfg["point_cloud_range"],
+                                                 cfg["max_points"], cfg["max_voxels"], 0)
+        bev, bev_h16 = None, None
+        if self.keep_bev:
+            bev = self.net(mean, coors, 1, num=nv)
+            h = self.dense(bev) if self.dense is not None else self.head
+        else:
+            bev_h16 = self.net(mean, coors, 1, num=nv, pixel_h16=True)
+            h = self.dense.forward_h16(*bev_h16)
+        # frame status word (ADVICE r1): [fp16-range overflow of the pair-row kernels, overflow flag of each strided level]
+        status = torch.stack([sp.status_tensor(self.device)[0]] + [c[1] for c in self.net.level_counters])
+        boxes, scores, labels, counts = cpp.centerpoint_postprocess_device(
+            h["hm"], h["reg"], h["height"], h["dim"], h["vel"], h["rot"], cfg["voxel_size"][:2],
+            cfg["point_cloud_range"], tc["post_center_limit_range"], self.label_off, tc["down_ratio"],
+            tc["score_threshold"], tc["nms_iou_threshold"], tc["nms_pre_max_size"], tc["nms_post_max_size"], True)
+        return dict(bev=bev, bev_h16=bev_h16, boxes=boxes, scores=scores, labels=labels, counts=counts, num_voxels=nv,
+                    coors=coors, mean=mean, status=status)
+
+    def bev_nchw(self):
+        """The dense BEV tensor [1, 256, H, W] fp32 of the last frame (rebuilt from the pixel fp16-pair image when the
+        frame did not materialise it)."""
+        if self.out["bev"] is not None:
+            self.stream.synchronize()
+            return self.out["bev"]
+        from .ops import dense_conv as dc
+        rows, shape = self.out["bev_h16"]
+        with torch.cuda.stream(self.stream):
+            out = dc.pixel_h16_to_nchw(rows, shape)
+            # pixel rows hold (z, c)-ordered channels (to_pixel_h16); the reference tensor is (c, z)-ordered
+            b, h, w, cd = shape
+            D = self.dense.bev_depth
+            out = out.view(b, D, cd // D, h, w).transpose(1, 2).reshape(b, cd, h, w).contiguous()
+        self.stream.synchronize()  # callers read it from other streams
+        return out
+
+    def calibrate_head(self, points_dev):
+        """Shift the heat-map biases of the (randomly initialised) dense head so that ~1.4 % of the BEV cells of this frame
+        score above the threshold, as SURVEY.md §8d specifies for the synthetic workload (see
+        DenseRPNHead.calibrate_heatmap_bias).  Call before capture()."""
+        if self.dense is None:
+            return self
+        cfg = self.cfg
+        with torch.cuda.stream(self.stream):
+            self.points.copy_(points_dev)
+            mean, coors, npv, nv = vox.voxelize_mean(self.points, cfg["voxel_size"], cfg["point_cloud_range"],
+                                                     cfg["max_points"], cfg["max_voxels"], 0)
+            bev = self.net(mean, coors, 1, num=nv)
+            self.dense.calibrate_heatmap_bias(bev, self.test_cfg["score_threshold"])
+        self.stream.synchronize()
+        return self
+
+    @staticmethod
+    def check_status(status_host):
+        """Raise when the frame's device status word reports dropped work (never a silent wrong result)."""
+        st = [int(v) for v in status_host]
+        if st[0]:
+            raise RuntimeError("sparse backbone: an activation left fp16's range (|x| >= 65504) on the fp16-pair path; "
+                               "run this model with precision TF32X3_SPLIT")
+        for lvl, v in enumerate(st[1:]):
+            if v:
+                raise RuntimeError("sparse backbone: strided level %d overflowed its row capacity (set_level_caps); "
+                                   "output sites were dropped" % (lvl + 1))
+
     def export_weights_numpy(self):
         """Weights as plain numpy dicts for the CPU arm (oracle.cpu_reference.CpuFrame)."""
         def conv(l):
@@ -277,6 +295,86 @@ class CenterPointHotPath:
                     extra=dict(conv=conv(n.extra_conv[0]), bn=bn(n.extra_conv[1])))
 
 
+class CenterPointPillarsHotPath(_FramePipeline):
+    """CenterPoint-pillars hot-path frame (centerpoint_pillars_02voxel_nuscenes_10sweep.yml, synth.CP_PILLARS):
+
+        hard_voxelize -> PillarFeatureNet written straight into the pixel fp16-pair BEV image [1, 512, 512, 64]
+        -> SecondBackbone + SecondFPN (down-sampling, 1x1 and up-sampling deblocks) + CenterHead -> centerpoint_postprocess
+
+    captured as one CUDA graph, with the same public calls as CenterPointHotPath.  No fp32 NCHW canvas exists in the frame
+    (bev_nchw() rebuilds it on demand).  Status word: [fp16-range overflow of the pair-image kernels]."""
+
+    def __init__(self, cfg=None, device="cuda:0", seed=0, num_points=None, bn_gain=PILLARS_BN_GAIN, test_cfg=None):
+        from .dense_head import DenseRPNHead
+        from .layers import PillarFeatureNet, _grid
+        self.cfg = dict(cfg or synth.CP_PILLARS)
+        cfg = self.cfg
+        self.device = torch.device(device)
+        self.n = int(num_points or cfg["num_points"])
+        self.F = cfg["point_dim"]
+        self.test_cfg = dict(test_cfg or synth.CP_PILLARS_TEST_CFG)
+        self.label_off = synth.label_offsets()
+        g = _grid(cfg["point_cloud_range"], cfg["voxel_size"])
+        self.nx, self.ny = int(g[0]), int(g[1])
+        self.net = PillarFeatureNet(self.F, (cfg["pfn_channels"],), False, cfg["max_points"], cfg["voxel_size"],
+                                    cfg["point_cloud_range"])
+        self.net.init_weight(seed=seed, device=self.device, bn_gain=bn_gain)
+        self.dense = DenseRPNHead(**cfg["backbone"]).init_weight(seed=seed + 1, device=self.device, bn_gain=bn_gain)
+        self._init_io(1)
+
+    def _front(self):
+        """hard_voxelize + the pillar encoder into the pixel fp16-pair image: (rows, shape), num_voxels, coors."""
+        cfg = self.cfg
+        voxels, coords, npv, nv = vox.hard_voxelize(self.points, cfg["voxel_size"], cfg["point_cloud_range"],
+                                                    cfg["max_points"], cfg["max_voxels"])
+        coors = torch.nn.functional.pad(coords, (1, 0), value=0)  # (b, z, y, x), batch 0 (voxelize.py:51-57)
+        img = self.net.forward_pixel_h16(voxels, npv, coors, 1, self.ny, self.nx, num=nv)
+        return img, nv, coors
+
+    # ---- one frame, enqueued on the current stream, device in / device out
+    def forward_device(self):
+        cfg, tc = self.cfg, self.test_cfg
+        bev_h16, nv, coors = self._front()
+        h = self.dense.forward_h16(*bev_h16)
+        status = sp.status_tensor(self.device).clone()
+        boxes, scores, labels, counts = cpp.centerpoint_postprocess_device(
+            h["hm"], h["reg"], h["height"], h["dim"], h["vel"], h["rot"], cfg["voxel_size"][:2],
+            cfg["point_cloud_range"], tc["post_center_limit_range"], self.label_off, tc["down_ratio"],
+            tc["score_threshold"], tc["nms_iou_threshold"], tc["nms_pre_max_size"], tc["nms_post_max_size"], True)
+        return dict(bev=None, bev_h16=bev_h16, head=h, boxes=boxes, scores=scores, labels=labels, counts=counts,
+                    num_voxels=nv, coors=coors, status=status)
+
+    def bev_nchw(self):
+        """The pillar canvas [1, C, ny, nx] fp32 of the last frame, rebuilt from its pixel fp16-pair image."""
+        from .ops import dense_conv as dc
+        with torch.cuda.stream(self.stream):
+            out = dc.pixel_h16_to_nchw(*self.out["bev_h16"])
+        self.stream.synchronize()  # callers read it from other streams
+        return out
+
+    def calibrate_head(self, points_dev):
+        """As CenterPointHotPath.calibrate_head: shift the heat-map biases so that ~1.4 % of the cells of this frame score
+        above the threshold.  Call before capture()."""
+        from .ops import dense_conv as dc
+        with torch.cuda.stream(self.stream):
+            self.points.copy_(points_dev)
+            img, _, _ = self._front()
+            self.dense.calibrate_heatmap_bias(dc.pixel_h16_to_nchw(*img), self.test_cfg["score_threshold"])
+        self.stream.synchronize()
+        return self
+
+    @staticmethod
+    def check_status(status_host):
+        """Raise when the frame's device status word reports a saturated value (never a silent wrong result)."""
+        if int(status_host[0]):
+            raise RuntimeError("pillar frame: an activation left fp16's range (|x| > 65504) on the fp16-pair path and "
+                               "was saturated")
+
+    def export_weights_numpy(self):
+        """Weights as plain numpy dicts for the CPU arm (oracle.cpu_reference.CpuPillarFrame)."""
+        return dict(pfn=dict(self.net.np), dense=self.dense.export_numpy())
+
+
 class CenterPointSweep:
     """Several frames of a sweep in flight on ONE GPU.
 
@@ -288,13 +386,14 @@ class CenterPointSweep:
     of one frame does not improve (use CenterPointHotPath.infer for that); results are those of the single-lane pipeline.
     """
 
-    def __init__(self, lanes=2, **kw):
+    def __init__(self, lanes=2, pipeline_cls=CenterPointHotPath, **kw):
+        """pipeline_cls: CenterPointHotPath or CenterPointPillarsHotPath; kw go to its constructor."""
         if lanes < 1:
             raise ValueError("lanes >= 1")
-        first = CenterPointHotPath(**kw)
+        first = pipeline_cls(**kw)
         self.lanes = [first]
         for _ in range(lanes - 1):
-            p = CenterPointHotPath(**kw)
+            p = pipeline_cls(**kw)
             p.net, p.dense = first.net, first.dense  # one model: calibration / weight loading happens once, on lane 0
             self.lanes.append(p)
         self.device = first.device

@@ -27,6 +27,15 @@ CENTERPOINT_TASKS = [1, 2, 2, 1, 2, 2]  # classes per task (yml:139-151)
 CENTERPOINT_TEST_CFG = dict(  # yml:163-172
     post_center_limit_range=[-61.2, -61.2, -10.0, 61.2, 61.2, 10.0], nms_pre_max_size=1000, nms_post_max_size=83,
     nms_iou_threshold=0.2, score_threshold=0.1, down_ratio=8)
+# configs/centerpoint/centerpoint_pillars_02voxel_nuscenes_10sweep.yml: 0.2 m pillars on a 512 x 512 grid, one PFN layer
+# of 64 channels, SecondBackbone 64/128/256 (layer_nums 3/5/5, strides 2/2/2), SecondFPN 128 x 3 with upsample_strides
+# [0.5, 1, 2] (concat 384 channels at 128 x 128), CenterHead as the voxel model's; head maps at stride 4
+CP_PILLARS = dict(name="centerpoint_pillar_02", num_points=300000, point_dim=5, voxel_size=[0.2, 0.2, 8.0],
+                  point_cloud_range=[-51.2, -51.2, -5.0, 51.2, 51.2, 3.0], max_points=20, max_voxels=40000,
+                  pfn_channels=64, backbone=dict(in_channels=64, out_channels=(64, 128, 256), layer_nums=(3, 5, 5),
+                                                 downsample_strides=(2, 2, 2), fpn_out_channels=(128, 128, 128),
+                                                 upsample_strides=(0.5, 1, 2), share_conv_channel=64, bev_depth=1))
+CP_PILLARS_TEST_CFG = dict(CENTERPOINT_TEST_CFG, down_ratio=4)
 
 
 def uniform_cloud(cfg, seed, num_points=None, margin=0.02):
