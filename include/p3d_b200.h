@@ -140,6 +140,29 @@ int p3d_centerpoint_postprocess(int num_tasks, const float *const *hm, const int
                                 size_t workspace_bytes, p3d_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * anchor_head_postprocess      the SSD head's post-processing of PointPillars / SECOND (the reference runs it as Python
+ *                              over Paddle ops: pointpillars.py:105-129 + rotate_nms_pcdet), batch size 1.
+ *   cls [A*C, H, W], box [A*7, H, W], dir [A*2, H, W]: fp32 NCHW planes on the device; anchor i = (y * W + x) * A + a
+ *   reads cls[a*C + c], box[a*7 + k], dir[a*2 + d].  anchors [H*W*A, 7] (x, y, z, w, l, h, r) fp32 on the device.
+ *   Anchor mask (skipped when anchor_cells is NULL or anchor_area_threshold < 0): anchor_cells [H*W*A] int4 (x0, y0, x1,
+ *   y1) are the static clipped cell bounds of fused_get_anchors_area; the pillar occupancy of coors [num_voxels, 4]
+ *   (b, z, y, x) int32 on a grid_ny x grid_nx grid gives each anchor an area, and it is kept iff area > threshold.
+ *   Candidates: max sigmoid score >= score_threshold.  The first nms_pre_max_size in descending score order (ties: ascending
+ *   anchor index) are decoded (second_box_decode), suppressed by rotated NMS (rotate_nms_pcdet's box layout), cut to
+ *   nms_post_max_size, direction-fixed and filtered by post_center_range_host (6 floats, inclusive; NULL: no filter).
+ *   Outputs (device), sized for nms_post_max_size rows: boxes [., 7], scores, labels int64, anchor_index_out int32 (may be
+ *   NULL), counts [2] int32 = (candidates, rows).  No row is emitted when nothing passes.
+ * ------------------------------------------------------------------------------------------- */
+size_t p3d_anchor_head_postprocess_workspace_bytes(int num_anchors, int grid_ny, int grid_nx, int nms_pre_max_size);
+int p3d_anchor_head_postprocess(const float *cls, const float *box, const float *dir, int H, int W, int A, int C,
+                                const float *anchors, const int32_t *anchor_cells, const int32_t *coors,
+                                const int32_t *num_voxels_dev, int grid_ny, int grid_nx, float anchor_area_threshold,
+                                float score_threshold, float iou_threshold, int nms_pre_max_size, int nms_post_max_size,
+                                const float *post_center_range_host, float *boxes_out, float *scores_out,
+                                int64_t *labels_out, int32_t *anchor_index_out, int32_t *counts_out, void *workspace,
+                                size_t workspace_bytes, p3d_stream_t stream);
+
+/* ---------------------------------------------------------------------------------------------
  * Sparse 3-D convolution      replaces the paddle.sparse.nn layer calls made by SparseResNet3D /
  *   SparseNet3D (paddle3d/models/middle_encoders/sparse_resnet.py:31-60,84-111,125-206;
  *   sparsenet.py:38-52,75-155): SubmConv3D / Conv3D (+ BatchNorm(eval) + residual add + ReLU fused).

@@ -38,6 +38,9 @@ SIGNATURES = {
     "p3d_centerpoint_postprocess_workspace_bytes": (_sz, [_int, _int, _int, _int, _int]),
     "p3d_centerpoint_postprocess": (_int, [_int, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _int, _int, _vp, _vp, _vp, _vp,
                                            _int, _f, _f, _int, _int, _int, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "p3d_anchor_head_postprocess_workspace_bytes": (_sz, [_int, _int, _int, _int]),
+    "p3d_anchor_head_postprocess": (_int, [_vp, _vp, _vp, _int, _int, _int, _int, _vp, _vp, _vp, _vp, _int, _int, _f, _f,
+                                           _f, _int, _int, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "p3d_sparse_rulebook_workspace_bytes": (_sz, [_i64, _i64]),
     "p3d_sparse_rulebook_subm": (_int, [_vp, _vp, _i64, _int, _vp, _vp, _vp, _vp, _sz, _vp]),
     "p3d_sparse_rulebook_conv": (_int, [_vp, _vp, _i64, _int, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp, _vp, _sz,

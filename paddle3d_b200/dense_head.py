@@ -6,7 +6,8 @@ with BatchNorm folded into the conv epilogue.  Same constructor vocabulary as th
 pair operands on tcgen05 (csrc/dense_conv_f16.cu, `f16=True`); the round-1 tf32-pair kernels stay selectable
 (`f16=False`) for data outside fp16's range.  The 36 ConvModules of the heads run as ONE 64 -> 2304 convolution and
 the 36 output convs as one grouped CUDA-core launch (forward); forward_per_head keeps the layer-by-layer form for
-the parity tests."""
+the parity tests.  SecondRPN (backbone + FPN up to the concat) is the trunk DenseRPNHead and the PointPillars SSD head
+(anchor_head.SSDHead) share."""
 import os
 
 import numpy as np
@@ -79,19 +80,19 @@ class _Conv:
                                d["scale"], d["shift"], self.relu, **kw)
 
 
-class DenseRPNHead:
+class SecondRPN:
+    """SecondBackbone (second_backbone.py:72-120) + SecondFPN (second_fpn.py:99-160, use_conv_for_no_stride): the trunk both
+    heads run on, from the BEV image to the channel concat of the FPN levels (pixel fp16-pair rows on the default path).
+    DenseRPNHead initialises these convs within its own seeded stream (convs() first, then prepare()); a stand-alone trunk
+    uses init_weight."""
+
     def __init__(self, in_channels=256, out_channels=(128, 256), layer_nums=(5, 5), downsample_strides=(1, 2),
-                 fpn_out_channels=(256, 256), upsample_strides=(1, 2), tasks=(1, 2, 2, 1, 2, 2), share_conv_channel=64,
-                 f16=True, with_velocity=True, bev_depth=2):
-        self.tasks = list(tasks)
-        self.in_channels, self.bev_depth = in_channels, bev_depth
-        self.num_classes = list(tasks)        # CenterHead.num_classes (center_head.py:64)
-        self.with_velocity = with_velocity    # 'vel' in common_heads (center_head.py:77)
-        self.f16 = f16
+                 fpn_out_channels=(256, 256), upsample_strides=(1, 2), f16=True, bev_depth=2):
+        self.in_channels, self.bev_depth, self.f16 = in_channels, bev_depth, f16
 
         def conv(*a, **k):
             return _Conv(*a, f16=f16, **k)
-        bn3, bn5 = 1e-3, 1e-5
+        bn3 = 1e-3
         self.blocks = []
         cin = in_channels
         for cout, n, s in zip(out_channels, layer_nums, downsample_strides):
@@ -110,34 +111,21 @@ class DenseRPNHead:
                 k = int(round(1.0 / u))
                 self.deblocks.append(conv(ci, co, k, k, 0, bn_eps=bn3))
         self.fpn_channels = int(sum(fpn_out_channels))
-        self.shared = conv(self.fpn_channels, share_conv_channel, 3, 1, 1, bias=True, bn_eps=bn5)
-        self.heads = []  # per task: list of (name, ConvModule 64->64, final conv 64->classes)
-        for ncls in self.tasks:
-            hs = []
-            for name, c in list(COMMON_HEADS) + [("hm", ncls)]:
-                hs.append((name, conv(share_conv_channel, share_conv_channel, 3, 1, 1, bias=True, bn_eps=bn5),
-                           conv(share_conv_channel, c, 3, 1, 1, bias=True, relu=False)))
-            self.heads.append(hs)
-        self._batched = None
+        self._first_zc = None
 
-    def all_convs(self):
-        out = [c for blk in self.blocks for c in blk] + list(self.deblocks) + [self.shared]
-        for hs in self.heads:
-            for _, a, b in hs:
-                out += [a, b]
-        return out
+    def convs(self):
+        return [c for blk in self.blocks for c in blk] + list(self.deblocks)
 
     def init_weight(self, seed=0, device="cuda", randomize_bn=False, bn_gain=1.0):
-        """device=None: numpy parameters only (enough for export_numpy / the CPU arm).  bn_gain multiplies every BatchNorm
-        gamma (sqrt(6) keeps the activations O(1) through the stack, see sparse_nn.BatchNorm.init_parameters)."""
+        """Seeded parameters of a stand-alone trunk (as DenseRPNHead.init_weight does for its own convs)."""
         rng = np.random.default_rng(seed)
-        hm_finals = {id(b) for hs in self.heads for name, _, b in hs if name == "hm"}
-        finals = {id(b) for hs in self.heads for _, _, b in hs}
-        for c in self.all_convs():  # hm bias = -2.19 (center_head.py:113-117)
-            # the 1-3 channel output convs have no tensor-core image in f16 mode: they run grouped on the CUDA cores
-            dev = None if (self.f16 and id(c) in finals) else device
-            c.init(rng, dev, randomize_bn, bias_value=-2.19 if id(c) in hm_finals else None, bn_gain=bn_gain)
-        self._batched = None
+        for c in self.convs():
+            c.init(rng, device, randomize_bn, bn_gain=bn_gain)
+        return self.prepare(device)
+
+    def prepare(self, device):
+        """After the convs are initialised: the second image of the first conv for pixel fp16-pair input (forward with a
+        shape)."""
         self._first_zc = None
         if self.f16 and device is not None and self.in_channels % self.bev_depth == 0:
             # second image of the first conv for BEV tensors that arrive as pixel fp16-pair rows straight from the sparse
@@ -154,8 +142,7 @@ class DenseRPNHead:
         return self
 
     def export_numpy(self):
-        return dict(blocks=[[c.np for c in blk] for blk in self.blocks], deblocks=[c.np for c in self.deblocks],
-                    shared=self.shared.np, heads=[[(n, a.np, b.np) for n, a, b in hs] for hs in self.heads])
+        return dict(blocks=[[c.np for c in blk] for blk in self.blocks], deblocks=[c.np for c in self.deblocks])
 
     @staticmethod
     def deblock_out_hw(de, h, w):
@@ -172,9 +159,18 @@ class DenseRPNHead:
             raise ValueError("SecondFPN deblocks produce different sizes %s: they cannot be concatenated" % sizes)
         return sizes[0]
 
-    # ---- RPN + neck + shared conv: bev [B, C, H, W] fp32 -> (pixel rows of the shared feature map, its shape)
-    def _trunk(self, bev, shape=None):
-        """bev: fp32 NCHW tensor, or (shape given) pixel fp16-pair rows [B*H*W, 2*C] with shape = (B, H, W, C)."""
+    def out_hw(self, H, W):
+        """(H, W) of the concat for an H x W input."""
+        shapes = []
+        for blk in self.blocks:
+            for c in blk:
+                H, W = (H + 2 * c.padding - c.k) // c.stride + 1, (W + 2 * c.padding - c.k) // c.stride + 1
+            shapes.append((1, H, W, blk[-1].cout))
+        return self.fpn_out_hw(shapes)
+
+    def forward(self, bev, shape=None):
+        """bev: fp32 NCHW tensor, or (shape given) pixel fp16-pair rows [B*H*W, 2*C] with shape = (B, H, W, C).  Returns
+        (pixel rows of the FPN concat, (B, H, W, fpn_channels))."""
         first = None
         if shape is None:
             b, c, h, w = bev.shape
@@ -201,9 +197,75 @@ class DenseRPNHead:
         for (f, fshape), de in zip(feats, self.deblocks):
             de(f, fshape, out_split=cat, out_channels=self.fpn_channels, out_c0=c0)
             c0 += de.cout
-        H, W = out_hw
-        s, _, _ = self.shared(cat, (b, H, W, self.fpn_channels))
-        return s, (b, H, W, self.shared.cout)
+        return cat, (b, out_hw[0], out_hw[1], self.fpn_channels)
+
+    __call__ = forward
+
+
+class DenseRPNHead:
+    def __init__(self, in_channels=256, out_channels=(128, 256), layer_nums=(5, 5), downsample_strides=(1, 2),
+                 fpn_out_channels=(256, 256), upsample_strides=(1, 2), tasks=(1, 2, 2, 1, 2, 2), share_conv_channel=64,
+                 f16=True, with_velocity=True, bev_depth=2):
+        self.tasks = list(tasks)
+        self.in_channels, self.bev_depth = in_channels, bev_depth
+        self.num_classes = list(tasks)        # CenterHead.num_classes (center_head.py:64)
+        self.with_velocity = with_velocity    # 'vel' in common_heads (center_head.py:77)
+        self.f16 = f16
+
+        def conv(*a, **k):
+            return _Conv(*a, f16=f16, **k)
+        bn5 = 1e-5
+        self.rpn = SecondRPN(in_channels, out_channels, layer_nums, downsample_strides, fpn_out_channels, upsample_strides,
+                             f16, bev_depth)
+        self.blocks, self.deblocks, self.fpn_channels = self.rpn.blocks, self.rpn.deblocks, self.rpn.fpn_channels
+        self.shared = conv(self.fpn_channels, share_conv_channel, 3, 1, 1, bias=True, bn_eps=bn5)
+        self.heads = []  # per task: list of (name, ConvModule 64->64, final conv 64->classes)
+        for ncls in self.tasks:
+            hs = []
+            for name, c in list(COMMON_HEADS) + [("hm", ncls)]:
+                hs.append((name, conv(share_conv_channel, share_conv_channel, 3, 1, 1, bias=True, bn_eps=bn5),
+                           conv(share_conv_channel, c, 3, 1, 1, bias=True, relu=False)))
+            self.heads.append(hs)
+        self._batched = None
+
+    def all_convs(self):
+        out = self.rpn.convs() + [self.shared]
+        for hs in self.heads:
+            for _, a, b in hs:
+                out += [a, b]
+        return out
+
+    def init_weight(self, seed=0, device="cuda", randomize_bn=False, bn_gain=1.0):
+        """device=None: numpy parameters only (enough for export_numpy / the CPU arm).  bn_gain multiplies every BatchNorm
+        gamma (sqrt(6) keeps the activations O(1) through the stack, see sparse_nn.BatchNorm.init_parameters)."""
+        rng = np.random.default_rng(seed)
+        hm_finals = {id(b) for hs in self.heads for name, _, b in hs if name == "hm"}
+        finals = {id(b) for hs in self.heads for _, _, b in hs}
+        for c in self.all_convs():  # hm bias = -2.19 (center_head.py:113-117)
+            # the 1-3 channel output convs have no tensor-core image in f16 mode: they run grouped on the CUDA cores
+            dev = None if (self.f16 and id(c) in finals) else device
+            c.init(rng, dev, randomize_bn, bias_value=-2.19 if id(c) in hm_finals else None, bn_gain=bn_gain)
+        self._batched = None
+        self.rpn.prepare(device)
+        return self
+
+    def export_numpy(self):
+        return dict(self.rpn.export_numpy(), shared=self.shared.np,
+                    heads=[[(n, a.np, b.np) for n, a, b in hs] for hs in self.heads])
+
+    deblock_out_hw = staticmethod(SecondRPN.deblock_out_hw)
+
+    def fpn_out_hw(self, feat_shapes):
+        """(H, W) of the SecondFPN concat for backbone outputs of shapes (B, H, W, C); raises ValueError when the
+        deblocks bring the levels to different sizes."""
+        return self.rpn.fpn_out_hw(feat_shapes)
+
+    # ---- RPN + neck + shared conv: bev [B, C, H, W] fp32 -> (pixel rows of the shared feature map, its shape)
+    def _trunk(self, bev, shape=None):
+        """bev: fp32 NCHW tensor, or (shape given) pixel fp16-pair rows [B*H*W, 2*C] with shape = (B, H, W, C)."""
+        cat, shape = self.rpn(bev, shape)
+        s, _, _ = self.shared(cat, shape)
+        return s, shape[:3] + (self.shared.cout,)
 
     def _final_convs(self, mid, shape, in_C, groups_params, planes_total, device):
         """Grouped 64 -> {1..3} output convs in one launch: tensor cores on the fp16-pair path (p3d_grouped_head_conv_f16),

@@ -4,7 +4,7 @@
     Predictor(...).run(points)                      infer.py:163-189  -> (box3d_lidar [K, 9], label_preds [K], scores [K]) on the host
     parse_result(box3d_lidar, label_preds, scores)  infer.py:139-160  the reference's text format, fake rows (score -1) skipped
 
-The predictor is `CenterPointHotPath` (or, with pipeline_cls, `CenterPointPillarsHotPath`) behind the reference's three-output contract (the exported model's outputs are
+The predictor is `CenterPointHotPath` (or, with pipeline_cls, `CenterPointPillarsHotPath` / `PointPillarsHotPath`) behind the reference's three-output contract (the exported model's outputs are
 box3d_lidar, label_preds, scores in that order, infer.py:180-188).  A frame may hold fewer points than the capacity the
 pipeline was captured for: the tail of the device buffer is filled with NaN rows, which `hard_voxelize` drops exactly
 like the reference drops out-of-range points (voxelize_op.cc:37-45 -> csrc/voxelize.cu cell_of).  Host code, as in the
@@ -63,19 +63,19 @@ class Predictor:
 
     def __init__(self, cfg=None, device="cuda:0", max_points=None, seed=0, precision=None, with_head=True, weights=None,
                  pipeline_cls=None):
-        """pipeline_cls: CenterPointHotPath (default; cfg defaults to synth.C3) or CenterPointPillarsHotPath (cfg defaults
-        to synth.CP_PILLARS; precision and with_head do not apply: the pillar model always runs its fp16-pair dense head)."""
+        """pipeline_cls: CenterPointHotPath (default), CenterPointPillarsHotPath or PointPillarsHotPath; cfg defaults to the
+        class's default_cfg (synth.C3, synth.CP_PILLARS, synth.PP_KITTI_CAR).  precision and with_head apply to the voxel
+        model only: the pillar models always run their fp16-pair dense heads."""
         import torch
-        from . import synth
         from .ops import sparse_nn as sp
         from .pipeline import CenterPointHotPath
         self.torch = torch
-        if pipeline_cls is None or pipeline_cls is CenterPointHotPath:
-            self.cfg = dict(cfg or synth.C3)
+        pipeline_cls = pipeline_cls or CenterPointHotPath
+        self.cfg = dict(cfg or pipeline_cls.default_cfg)
+        if pipeline_cls is CenterPointHotPath:
             self.pipe = CenterPointHotPath(self.cfg, device, precision=sp.F16X3 if precision is None else precision,
                                            seed=seed, num_points=max_points, with_head=with_head)
         else:
-            self.cfg = dict(cfg or synth.CP_PILLARS)
             self.pipe = pipeline_cls(self.cfg, device, seed=seed, num_points=max_points)
         self.host = torch.empty((self.pipe.n, self.pipe.F), dtype=torch.float32).pin_memory()
         self.captured = False

@@ -1,6 +1,7 @@
 """CenterPoint hot-path frames on one B200: the public API a user calls (bench.py `e2e`).  CenterPointHotPath is the voxel
 model (below); CenterPointPillarsHotPath the 0.2 m pillar model (hard_voxelize -> PillarFeatureNet into the pixel fp16-pair
-BEV image -> the same dense RPN / neck / CenterHead -> centerpoint_postprocess).  Both share their frame I/O
+BEV image -> the same dense RPN / neck / CenterHead -> centerpoint_postprocess); PointPillarsHotPath the PointPillars KITTI
+car model (same pillar front end -> SecondRPN -> SSD head -> anchor_head_postprocess).  All share their frame I/O
 (_FramePipeline) and run side by side in CenterPointSweep lanes.
 
     voxelize (+ VoxelMean fused)  ->  SparseResNet3D (21 sparse convs)  ->  dense BEV [1,256,180,180]
@@ -53,17 +54,25 @@ class _FramePipeline:
     forward_device() (one frame enqueued on the current stream, returning a dict with at least boxes, scores, labels,
     counts and status) and check_status() (raises on a non-zero device status word)."""
 
-    def _init_io(self, status_words):
-        """Needs self.n, self.F, self.device, self.label_off and self.test_cfg."""
+    # attributes a CenterPointSweep lane shares with lane 0 (one model); default_cfg: the configuration a Predictor uses
+    shared_attrs = ("net", "dense")
+    default_cfg = None
+
+    def _init_io(self, status_words, rows=None, box_dim=9, count_words=None):
+        """Needs self.n, self.F, self.device, and (for the defaults of rows / count_words: one block of result rows and
+        one count per task, then the total) self.label_off and self.test_cfg.  The total row count is the last count."""
         self.points = torch.zeros((self.n, self.F), dtype=torch.float32, device=self.device)  # static input
         self.graph = None
         self.out = None
         self.stream = torch.cuda.Stream(self.device)
-        rows = len(self.label_off) * self.test_cfg["nms_post_max_size"]
-        self.h_boxes = torch.empty((rows, 9), dtype=torch.float32).pin_memory()
+        if rows is None:
+            rows = len(self.label_off) * self.test_cfg["nms_post_max_size"]
+        if count_words is None:
+            count_words = len(self.label_off) + 1
+        self.h_boxes = torch.empty((rows, box_dim), dtype=torch.float32).pin_memory()
         self.h_scores = torch.empty((rows,), dtype=torch.float32).pin_memory()
         self.h_labels = torch.empty((rows,), dtype=torch.int64).pin_memory()
-        self.h_counts = torch.empty((len(self.label_off) + 1,), dtype=torch.int32).pin_memory()
+        self.h_counts = torch.empty((count_words,), dtype=torch.int32).pin_memory()
         self.h_status = torch.zeros((status_words,), dtype=torch.int32).pin_memory()
 
     def capture(self, warmup=2, count_nodes=False):
@@ -182,6 +191,8 @@ class _FramePipeline:
 
 
 class CenterPointHotPath(_FramePipeline):
+    default_cfg = synth.C3
+
     def __init__(self, cfg=None, device="cuda:0", precision=sp.FP32, seed=0, num_points=None, level_caps=None,
                  head_seed=0, with_head=False, keep_bev=True, bn_gain=1.0):
         self.cfg = dict(cfg or synth.C3)
@@ -295,7 +306,36 @@ class CenterPointHotPath(_FramePipeline):
                     extra=dict(conv=conv(n.extra_conv[0]), bn=bn(n.extra_conv[1])))
 
 
-class CenterPointPillarsHotPath(_FramePipeline):
+class _PillarFramePipeline(_FramePipeline):
+    """Pillar front end shared by the pillar models: hard_voxelize + PillarFeatureNet written straight into the pixel
+    fp16-pair BEV image (needs self.cfg, self.net, self.ny, self.nx); status word [fp16-range overflow]."""
+
+    def _front(self):
+        """hard_voxelize + the pillar encoder into the pixel fp16-pair image: (rows, shape), num_voxels, coors."""
+        cfg = self.cfg
+        voxels, coords, npv, nv = vox.hard_voxelize(self.points, cfg["voxel_size"], cfg["point_cloud_range"],
+                                                    cfg["max_points"], cfg["max_voxels"])
+        coors = torch.nn.functional.pad(coords, (1, 0), value=0)  # (b, z, y, x), batch 0 (voxelize.py:51-57)
+        img = self.net.forward_pixel_h16(voxels, npv, coors, 1, self.ny, self.nx, num=nv)
+        return img, nv, coors
+
+    def bev_nchw(self):
+        """The pillar canvas [1, C, ny, nx] fp32 of the last frame, rebuilt from its pixel fp16-pair image."""
+        from .ops import dense_conv as dc
+        with torch.cuda.stream(self.stream):
+            out = dc.pixel_h16_to_nchw(*self.out["bev_h16"])
+        self.stream.synchronize()  # callers read it from other streams
+        return out
+
+    @staticmethod
+    def check_status(status_host):
+        """Raise when the frame's device status word reports a saturated value (never a silent wrong result)."""
+        if int(status_host[0]):
+            raise RuntimeError("pillar frame: an activation left fp16's range (|x| > 65504) on the fp16-pair path and "
+                               "was saturated")
+
+
+class CenterPointPillarsHotPath(_PillarFramePipeline):
     """CenterPoint-pillars hot-path frame (centerpoint_pillars_02voxel_nuscenes_10sweep.yml, synth.CP_PILLARS):
 
         hard_voxelize -> PillarFeatureNet written straight into the pixel fp16-pair BEV image [1, 512, 512, 64]
@@ -303,6 +343,7 @@ class CenterPointPillarsHotPath(_FramePipeline):
 
     captured as one CUDA graph, with the same public calls as CenterPointHotPath.  No fp32 NCHW canvas exists in the frame
     (bev_nchw() rebuilds it on demand).  Status word: [fp16-range overflow of the pair-image kernels]."""
+    default_cfg = synth.CP_PILLARS
 
     def __init__(self, cfg=None, device="cuda:0", seed=0, num_points=None, bn_gain=PILLARS_BN_GAIN, test_cfg=None):
         from .dense_head import DenseRPNHead
@@ -322,15 +363,6 @@ class CenterPointPillarsHotPath(_FramePipeline):
         self.dense = DenseRPNHead(**cfg["backbone"]).init_weight(seed=seed + 1, device=self.device, bn_gain=bn_gain)
         self._init_io(1)
 
-    def _front(self):
-        """hard_voxelize + the pillar encoder into the pixel fp16-pair image: (rows, shape), num_voxels, coors."""
-        cfg = self.cfg
-        voxels, coords, npv, nv = vox.hard_voxelize(self.points, cfg["voxel_size"], cfg["point_cloud_range"],
-                                                    cfg["max_points"], cfg["max_voxels"])
-        coors = torch.nn.functional.pad(coords, (1, 0), value=0)  # (b, z, y, x), batch 0 (voxelize.py:51-57)
-        img = self.net.forward_pixel_h16(voxels, npv, coors, 1, self.ny, self.nx, num=nv)
-        return img, nv, coors
-
     # ---- one frame, enqueued on the current stream, device in / device out
     def forward_device(self):
         cfg, tc = self.cfg, self.test_cfg
@@ -344,14 +376,6 @@ class CenterPointPillarsHotPath(_FramePipeline):
         return dict(bev=None, bev_h16=bev_h16, head=h, boxes=boxes, scores=scores, labels=labels, counts=counts,
                     num_voxels=nv, coors=coors, status=status)
 
-    def bev_nchw(self):
-        """The pillar canvas [1, C, ny, nx] fp32 of the last frame, rebuilt from its pixel fp16-pair image."""
-        from .ops import dense_conv as dc
-        with torch.cuda.stream(self.stream):
-            out = dc.pixel_h16_to_nchw(*self.out["bev_h16"])
-        self.stream.synchronize()  # callers read it from other streams
-        return out
-
     def calibrate_head(self, points_dev):
         """As CenterPointHotPath.calibrate_head: shift the heat-map biases so that ~1.4 % of the cells of this frame score
         above the threshold.  Call before capture()."""
@@ -363,16 +387,95 @@ class CenterPointPillarsHotPath(_FramePipeline):
         self.stream.synchronize()
         return self
 
-    @staticmethod
-    def check_status(status_host):
-        """Raise when the frame's device status word reports a saturated value (never a silent wrong result)."""
-        if int(status_host[0]):
-            raise RuntimeError("pillar frame: an activation left fp16's range (|x| > 65504) on the fp16-pair path and "
-                               "was saturated")
-
     def export_weights_numpy(self):
         """Weights as plain numpy dicts for the CPU arm (oracle.cpu_reference.CpuPillarFrame)."""
         return dict(pfn=dict(self.net.np), dense=self.dense.export_numpy())
+
+
+class PointPillarsHotPath(_PillarFramePipeline):
+    """PointPillars, KITTI car (synth.PP_KITTI_CAR; the reference's detection/pointpillars):
+
+        hard_voxelize -> PillarFeatureNet written straight into the pixel fp16-pair BEV image [1, 496, 432, 64]
+        -> SecondBackbone + SecondFPN (dense_head.SecondRPN: concat of 384 channels at 248 x 216)
+        -> SSD head (anchor_head.SSDHead: cls / box / dir as one 1x1 conv, 20 fp32 planes)
+        -> anchor_head_postprocess (anchor mask, scores, top-k, decode, rotated NMS, direction fix, range filter)
+
+    captured as one CUDA graph, with the same public calls as the CenterPoint pipelines.  Results: boxes [K, 7] (x, y, z,
+    w, l, h, r), scores [K], labels [K] (class index).  Status word: [fp16-range overflow of the pair-image kernels]."""
+    shared_attrs = ("net", "dense", "ssd")
+    default_cfg = synth.PP_KITTI_CAR
+
+    def __init__(self, cfg=None, device="cuda:0", seed=0, num_points=None, bn_gain=PILLARS_BN_GAIN, test_cfg=None):
+        from .anchor_head import SSDHead
+        from .dense_head import SecondRPN
+        from .layers import PillarFeatureNet, _grid
+        self.cfg = dict(cfg or synth.PP_KITTI_CAR)
+        cfg = self.cfg
+        self.device = torch.device(device)
+        self.n = int(num_points or cfg["num_points"])
+        self.F = cfg["point_dim"]
+        self.test_cfg = dict(test_cfg or cfg["test_cfg"])
+        g = _grid(cfg["point_cloud_range"], cfg["voxel_size"])
+        self.nx, self.ny = int(g[0]), int(g[1])
+        self.net = PillarFeatureNet(self.F, (cfg["pfn_channels"],), False, cfg["max_points"], cfg["voxel_size"],
+                                    cfg["point_cloud_range"])
+        self.net.init_weight(seed=seed, device=self.device, bn_gain=bn_gain)
+        self.dense = SecondRPN(**cfg["backbone"]).init_weight(seed=seed + 1, device=self.device, bn_gain=bn_gain)
+        fh, fw = self.dense.out_hw(self.ny, self.nx)
+        if tuple(cfg["anchors"]["feature_size"]) != (fh, fw):
+            raise ValueError("anchor feature_size %s does not match the FPN output %s" % (cfg["anchors"]["feature_size"],
+                                                                                         (fh, fw)))
+        self.ssd = SSDHead(self.dense.fpn_channels, cfg["num_classes"], cfg["anchors"]).init_weight(seed + 2, self.device)
+        self.ssd.set_mask_grid(cfg["voxel_size"], cfg["point_cloud_range"], (self.nx, self.ny))
+        self._init_io(1, rows=max(int(self.test_cfg["nms_post_max_size"]), 1), box_dim=7, count_words=2)
+
+    def _head(self, img):
+        """SecondRPN + the SSD conv on the pixel image: (cls, box, dir) fp32 NCHW views."""
+        cat, shape = self.dense(*img)
+        return self.ssd(cat, shape)
+
+    def _postprocess(self, head, coors, nv):
+        from .ops import anchor_head as ah
+        tc = self.test_cfg
+        return ah.anchor_head_postprocess_device(
+            head[0], head[1], head[2], self.ssd.anchors_dev, self.ssd.cells_dev, coors, nv, self.ny, self.nx,
+            tc["anchor_area_threshold"], tc["score_threshold"], tc["nms_iou_threshold"], tc["nms_pre_max_size"],
+            tc["nms_post_max_size"], tc["post_center_range"])
+
+    # ---- one frame, enqueued on the current stream, device in / device out
+    def forward_device(self):
+        bev_h16, nv, coors = self._front()
+        head = self._head(bev_h16)
+        status = sp.status_tensor(self.device).clone()
+        boxes, scores, labels, index, counts = self._postprocess(head, coors, nv)
+        return dict(bev=None, bev_h16=bev_h16, head=dict(cls=head[0], box=head[1], dir=head[2]), boxes=boxes,
+                    scores=scores, labels=labels, anchor_index=index, counts=counts, num_voxels=nv, coors=coors,
+                    status=status)
+
+    def anchor_mask(self, coors, num_voxels):
+        """The anchor mask of a frame on the host (bool [num_anchors]; None when the test config disables it)."""
+        from . import anchor_head
+        thr = self.test_cfg["anchor_area_threshold"]
+        if thr < 0:
+            return None
+        occ = anchor_head.occupancy(coors, num_voxels, self.ny, self.nx)
+        return anchor_head.anchors_area(occ, self.ssd.cells) > thr
+
+    def calibrate_head(self, points_dev):
+        """Shift the cls biases of the (seeded) SSD head so that ~1.4 % of the anchors score above the threshold on this
+        frame (SSDHead.calibrate_cls_bias; about 1 500 candidates, more than nms_pre_max_size).  Call before capture()."""
+        with torch.cuda.stream(self.stream):
+            self.points.copy_(points_dev)
+            img, nv, coors = self._front()
+            cat, shape = self.dense(*img)
+            keep = self.anchor_mask(coors.cpu().numpy(), int(nv.item()))
+            self.ssd.calibrate_cls_bias(cat, shape, self.test_cfg["score_threshold"], keep=keep)
+        self.stream.synchronize()
+        return self
+
+    def export_weights_numpy(self):
+        """Weights as plain numpy dicts for the CPU arm (tests/cpu_pointpillars_frame.py)."""
+        return dict(pfn=dict(self.net.np), dense=self.dense.export_numpy(), ssd=self.ssd.export_numpy())
 
 
 class CenterPointSweep:
@@ -387,14 +490,15 @@ class CenterPointSweep:
     """
 
     def __init__(self, lanes=2, pipeline_cls=CenterPointHotPath, **kw):
-        """pipeline_cls: CenterPointHotPath or CenterPointPillarsHotPath; kw go to its constructor."""
+        """pipeline_cls: CenterPointHotPath, CenterPointPillarsHotPath or PointPillarsHotPath; kw go to its constructor."""
         if lanes < 1:
             raise ValueError("lanes >= 1")
         first = pipeline_cls(**kw)
         self.lanes = [first]
         for _ in range(lanes - 1):
             p = pipeline_cls(**kw)
-            p.net, p.dense = first.net, first.dense  # one model: calibration / weight loading happens once, on lane 0
+            for name in pipeline_cls.shared_attrs:  # one model: calibration / weight loading happens once, on lane 0
+                setattr(p, name, getattr(first, name))
             self.lanes.append(p)
         self.device = first.device
 

@@ -36,6 +36,21 @@ CP_PILLARS = dict(name="centerpoint_pillar_02", num_points=300000, point_dim=5, 
                                                  downsample_strides=(2, 2, 2), fpn_out_channels=(128, 128, 128),
                                                  upsample_strides=(0.5, 1, 2), share_conv_channel=64, bev_depth=1))
 CP_PILLARS_TEST_CFG = dict(CENTERPOINT_TEST_CFG, down_ratio=4)
+# PointPillars, KITTI car (C2's voxelizer): one PFN layer of 64 channels, SecondBackbone 64/128/256 (layer_nums 3/5/5,
+# strides 2/2/2), SecondFPN 128 x 3 with upsample_strides [1, 2, 4] (concat 384 channels at 248 x 216), SSD head with 2
+# anchors per location and 1 class.  The anchor and test values are the standard PointPillars car ones (second.pytorch
+# car config); they were NOT re-read from the reference yml (DESIGN.md, known gaps).
+PP_KITTI_CAR = dict(C2, name="pointpillars_kitti_car", pfn_channels=64,
+                    backbone=dict(in_channels=64, out_channels=(64, 128, 256), layer_nums=(3, 5, 5),
+                                  downsample_strides=(2, 2, 2), fpn_out_channels=(128, 128, 128), upsample_strides=(1, 2, 4),
+                                  bev_depth=1),
+                    num_classes=1,
+                    # create_anchors_3d_stride: feature map (ny, nx), (w, l, h), x / y / z strides and offsets; rotations as
+                    # written in the config (1.57, not pi / 2)
+                    anchors=dict(feature_size=(248, 216), sizes=(1.6, 3.9, 1.56), strides=(0.32, 0.32, 0.0),
+                                 offsets=(0.16, -39.52, -1.78), rotations=(0, 1.57)),
+                    test_cfg=dict(score_threshold=0.05, nms_pre_max_size=1000, nms_post_max_size=300, nms_iou_threshold=0.5,
+                                  anchor_area_threshold=1, post_center_range=[0, -39.68, -5, 69.12, 39.68, 5]))
 
 
 def uniform_cloud(cfg, seed, num_points=None, margin=0.02):
